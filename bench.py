@@ -6,6 +6,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W                      # N > 1: per-sample sharding + ONE all-gather per step
     python bench.py --workload detr_r50|lxmert|clip_l14_336         # one of the other BASELINE configs as the main line
+    python bench.py --steps 5 --dump-outputs DIR                    # + the maps of the last timed step as DIR/<name>.npy
 
 Headline workload: a "step" = one interpret() pass over one batch of 64 synthetic (image, text) pairs PER GPU (weak
 scaling), all 12+12 blocks (start_layer = start_layer_text = 0: forward staging every A_l, dgrad-only backward staging
@@ -126,6 +127,25 @@ def workload_config(world: int, B: int, cfg) -> dict:
             "l2": "no flush: per-step working set (1.2 GB weights + >2 GB staged activations) >> 126 MB L2"}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """`--dump-outputs`: every array as `out_dir/<name>.npy` in float32.  All arrays lead with the sample dimension; above
+    DUMP_LIMIT_BYTES in all, the same seeded sample of samples (sorted indices) is kept from each."""
+    import numpy as np
+    arrays = {k: np.ascontiguousarray(v.detach().cpu().numpy() if hasattr(v, "detach") else v, dtype=np.float32)
+              for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        n = min(a.shape[0] for a in arrays.values())
+        keep = np.sort(np.random.default_rng(0).choice(n, max(1, n * DUMP_LIMIT_BYTES // total), replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 class ClockSampler(threading.Thread):
     """nvidia-smi clocks / throttle reasons DURING the timed region."""
 
@@ -186,9 +206,10 @@ def pick_threads() -> int:
     return best
 
 
-def cpu_baseline_run(batch: int, reps: int, warm: int, threads: int, start_layer: int = START_LAYER):
+def cpu_baseline_run(batch: int, reps: int, warm: int, threads: int, start_layer: int = START_LAYER, outputs=None):
     """The reference's own CPU PyTorch path, restated: per-block autograd.grad exactly like the notebook, the SAME
-    synthetic batch rank 0 of our arm processes (seed 1234, shared length multiset).  Returns (maps_per_s, median s)."""
+    synthetic batch rank 0 of our arm processes (seed 1234, shared length multiset).  Returns (maps_per_s, median s);
+    the maps of the last step go into ``outputs`` when given."""
     import torch
     import mmx_b200
     from oracle import clip_oracle as co
@@ -200,9 +221,11 @@ def cpu_baseline_run(batch: int, reps: int, warm: int, threads: int, start_layer
     ts = []
     for i in range(warm + reps):
         t0 = time.perf_counter()
-        co.clip_interpret(sd, cfg, images, tokens, start_layer, start_layer, per_layer_grad=True)
+        maps = co.clip_interpret(sd, cfg, images, tokens, start_layer, start_layer, per_layer_grad=True)
         if i >= warm:
             ts.append(time.perf_counter() - t0)
+    if outputs is not None:
+        outputs.update(R_text=maps[0], R_image=maps[1])
     ts.sort()
     med = ts[len(ts) // 2]
     return batch / med, med
@@ -216,7 +239,8 @@ def run_reference(args):
     threads = pick_threads()
     batch = BATCH_PER_GPU          # one step = the whole per-GPU batch of the workload, both arms the same config
     t_all0 = time.perf_counter()
-    val, sec = cpu_baseline_run(batch, max(1, args.steps), max(0, args.warmup), threads)
+    outputs = {}
+    val, sec = cpu_baseline_run(batch, args.steps, max(0, args.warmup), threads, outputs=outputs)
     val_def, sec_def = cpu_baseline_run(batch, 2, 1, threads, start_layer=-1)
     out = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -233,6 +257,8 @@ def run_reference(args):
         "e2e": {"value": val, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0, "wall_s": time.perf_counter() - t_all0,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(out), flush=True)
 
 
@@ -298,9 +324,11 @@ def timed_loop(D: Dist, step, finish, steps: int, warm: int, lib):
     return e0.elapsed_time(e1) / steps, lib.mmx_launch_count() - l0
 
 
-def bench_clip(D: Dist, cfg, B: int, steps: int, warm: int, max_batch: int, with_default: bool, with_check: bool, e2e_steps: int):
+def bench_clip(D: Dist, cfg, B: int, steps: int, warm: int, max_batch: int, with_default: bool, with_check: bool, e2e_steps: int,
+               outputs=None):
     """CLIP interpret() for B pairs per GPU: device-timed value, e2e through host buffers, per-rank times, the collective
-    alone, and (N > 1) the bitwise sharded == single-GPU check."""
+    alone, and (N > 1) the bitwise sharded == single-GPU check.  The maps of the last timed step (all ranks' after the
+    all-gather) go into ``outputs`` when given."""
     import mmx_b200
     from mmx_b200.distributed import gather_maps_packed, split_packed
     torch, dist = D.torch, D.dist
@@ -317,6 +345,7 @@ def bench_clip(D: Dist, cfg, B: int, steps: int, warm: int, max_batch: int, with
     n_total = B * world
     ctx, sv = cfg.context_length, cfg.vision_tokens
     pending = []
+    last = {}
 
     # The one collective of the path: ONE all-gather of the packed maps per step.  In stream order by default; with
     # MMX_BENCH_GATHER=async it overlaps the next step's forward - measured SLOWER at N = 2 (8.72 vs 7.95 ms per step): while
@@ -327,13 +356,15 @@ def bench_clip(D: Dist, cfg, B: int, steps: int, warm: int, max_batch: int, with
     def step_fn(sl):
         def step():
             rt, ri = eng.interpret(d_images, d_tokens, sl, sl, validate=False)
+            last["maps"] = rt, ri
             if world > 1:
                 if gather_async:
                     pending.append(gather_maps_packed(rt, ri, n_total, async_op=True))
+                    last["full"] = pending[-1][1]
                     while len(pending) > 2:
                         pending.pop(0)[0].wait()
                 else:
-                    gather_maps_packed(rt, ri, n_total, async_op=False)
+                    last["full"] = gather_maps_packed(rt, ri, n_total, async_op=False)[1]
             return rt, ri
         return step
 
@@ -346,6 +377,9 @@ def bench_clip(D: Dist, cfg, B: int, steps: int, warm: int, max_batch: int, with
         sampler.start()
     ms_rank, launches = timed_loop(D, step_fn(START_LAYER), finish, steps, warm, lib)
     clocks = sampler.stop() if sampler else None
+    if outputs is not None:
+        rt, ri = split_packed(last["full"], ctx, sv - 1) if world > 1 else last["maps"]
+        outputs.update(R_text=rt.cpu(), R_image=ri.cpu())
     per_rank = D.gather_floats(ms_rank)
     ms_step = max(per_rank)
     res = {"ms_per_step": ms_step, "value": n_total / (ms_step * 1e-3), "launches": int(launches), "clocks": clocks,
@@ -569,7 +603,7 @@ def _gemm_profile(lib, call, reps: int = 2):
     return tms.value / reps, tfl.value / reps, nl.value // reps
 
 
-def bench_detr(D: Dist, B: int, steps: int, warm: int):
+def bench_detr(D: Dist, B: int, steps: int, warm: int, outputs=None):
     """BASELINE config 3: DETR-R50 transformer (d 256, 8 heads, 6+6 layers, 100 queries) on 25x25 backbone features
     (625 tokens), B (image, query) pairs per GPU: Generator.generate_ours(use_lrp=False) (DETR/modules/
     ExplanationGenerator.py:142-195) captured once and replayed as a CUDA graph."""
@@ -587,6 +621,9 @@ def bench_detr(D: Dist, B: int, steps: int, warm: int):
     t_eager = _time_graph(D, lambda: gen.generate_ours((args[0], args[1]), args[2], use_lrp=False), max(2, steps // 2), 1)
     g = gen.capture((args[0], args[1]), args[2], use_lrp=False)
     ms = _time_graph(D, lambda: g(*args), steps, warm)
+    if outputs is not None:
+        (rel,) = g.outputs()
+        outputs["relevance"] = rel.cpu()
     g.check()
     same = bool(torch.equal(g(*args), eager_out))
     # e2e: pinned host features in, the target query's relevance rows out
@@ -623,7 +660,7 @@ def bench_detr(D: Dist, B: int, steps: int, warm: int):
                          "note": "eager tape, per-launch CUDA events on one stream"}}
 
 
-def bench_lxmert(D: Dist, B: int, steps: int, warm: int):
+def bench_lxmert(D: Dist, B: int, steps: int, warm: int, outputs=None):
     """BASELINE config 4: LXMERT base (768 hidden, 12 heads, 9/5/5 layers), 20 tokens x 36 boxes, B questions per GPU:
     GeneratorOurs.generate_ours(use_lrp=False) (lxmert/lxmert/src/ExplanationGenerator.py:131-211) as a CUDA graph."""
     import mmx_b200
@@ -640,6 +677,9 @@ def bench_lxmert(D: Dist, B: int, steps: int, warm: int):
     t_eager = _time_graph(D, lambda: gen.generate_ours(args, use_lrp=False), max(2, steps // 2), 1)
     g = gen.capture(args, use_lrp=False)
     ms = _time_graph(D, lambda: g(*args), steps, warm)
+    if outputs is not None:
+        r_tt, r_ti = g.outputs()
+        outputs.update(R_t_t=r_tt.cpu(), R_t_i=r_ti.cpu())
     g.check()
     o_tt, o_ti = g(*args)
     same = bool(torch.equal(o_tt, e_tt) and torch.equal(o_ti, e_ti))
@@ -678,11 +718,12 @@ def bench_lxmert(D: Dist, B: int, steps: int, warm: int):
                          "note": "eager tape, per-launch CUDA events on one stream"}}
 
 
-def bench_l14(D: Dist, B: int, steps: int, warm: int):
+def bench_l14(D: Dist, B: int, steps: int, warm: int, outputs=None):
     """BASELINE config 5: CLIP ViT-L/14@336, B pairs per GPU (2048 over 8 GPUs = 256 per GPU), micro-batches of 64."""
     import mmx_b200
     cfg = mmx_b200.VIT_L14_336
-    res, eng, inputs = bench_clip(D, cfg, B, steps, warm, max_batch=64, with_default=False, with_check=False, e2e_steps=max(1, steps // 2))
+    res, eng, inputs = bench_clip(D, cfg, B, steps, warm, max_batch=64, with_default=False, with_check=False, e2e_steps=max(1, steps // 2),
+                                  outputs=outputs)
     lib = mmx_b200.lib()
     eng.set_serial(True)
     gemm_ms, gemm_fl, gemm_n = _gemm_profile(lib, lambda: eng.interpret(inputs[0], inputs[1], START_LAYER, START_LAYER, validate=False), reps=1)
@@ -712,7 +753,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the short runs of the other BASELINE configs")
     ap.add_argument("--batch", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the maps of the last timed step as DIR/<name>.npy (float32; seeded inputs, so runs compare)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -722,19 +767,23 @@ def main():
     world, rank = D.world, D.rank
     warm = max(3, args.warmup)
     lib = mmx_b200.lib()
+    outputs = {} if args.dump_outputs and rank == 0 else None
 
     if args.workload != "clip_b32":                       # one of the other configs as the main (and only) line
         fn, Bdef = {"detr_r50": (bench_detr, 16), "lxmert": (bench_lxmert, 16), "clip_l14_336": (bench_l14, 256)}[args.workload]
-        r = fn(D, args.batch or Bdef, args.steps, warm)
+        r = fn(D, args.batch or Bdef, args.steps, warm, outputs=outputs)
         if rank == 0:
             r.update({"metric": "relevancy maps/sec (" + r["config"]["workload"] + ")", "n_gpus": world, "higher_is_better": True,
                       "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic"})
+            if outputs is not None:
+                dump_outputs(args.dump_outputs, outputs)
             print(json.dumps(r), flush=True)
         return D.close()
 
     B = args.batch or BATCH_PER_GPU
     cfg = mmx_b200.VIT_B32
-    res, eng, inputs = bench_clip(D, cfg, B, args.steps, warm, max_batch=B, with_default=True, with_check=True, e2e_steps=args.steps)
+    res, eng, inputs = bench_clip(D, cfg, B, args.steps, warm, max_batch=B, with_default=True, with_check=True, e2e_steps=args.steps,
+                                  outputs=outputs)
     roofline = clip_roofline(D, eng, inputs, B, cfg)
     roofline_rule5 = rule5_roofline(D, cfg, B)
     eager = None
@@ -777,6 +826,8 @@ def main():
         for k in ("collective", "sharded_equals_single"):
             if k in res:
                 out[k] = res[k]
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(out), flush=True)
     D.close()
 

@@ -11,8 +11,8 @@ the oracle is pinned against *outputs of the reference itself run in the build c
 ``oracle/make_golden.py`` imports the unmodified reference from ``/root/reference`` (with the import shims
 of ``oracle/ref_shims.py``), runs it on seeded inputs and commits the results under ``tests/golden/``.
 ``tests/test_oracle_golden.py`` checks this restatement against those fixtures everywhere, and
-``tests/test_oracle_vs_reference.py`` re-checks it against the live reference whenever ``/root/reference``
-is present.  Nothing on the path is unpinned any more (round 2): the ViT-B/16 *model* forward - whose source is not
+``tests/test_oracle_vs_reference.py`` at wider shapes (ViT-B/32 full size; fixture ``oracle_vs_reference.npz``).
+Nothing on the path is unpinned any more (round 2): the ViT-B/16 *model* forward - whose source is not
 vendored in the reference tree, SURVEY.md §8c - is pinned against torchvision's ``VisionTransformer`` with shared weights
 (``tests/test_vit_pin.py``: logits and every block's attention probabilities), the VisualBERT *embeddings* run the
 reference's own ``BertVisioLinguisticEmbeddings`` class loaded by file path (``ref_visualbert._import_embeddings``), and

@@ -249,9 +249,54 @@ def golden_visualbert():
     print("wrote visualbert_tiny", out["R.ours"].shape)
 
 
+def golden_vs_reference():
+    """The cases of tests/test_oracle_vs_reference.py at shapes wider than the fixtures above (ViT-B/32 full size, a
+    VisualBERT / DETR / LXMERT wider than the tiny configs).  Weights and inputs come from the seeded generators the test
+    calls again, so only the reference outputs are stored."""
+    from . import detr_oracle as do, lxmert_oracle as lo, visualbert_oracle as vo, ref_detr, ref_lxmert, ref_visualbert
+    out = {}
+    cfg = co.VIT_B32
+    sd = co.init_state_dict(cfg, seed=0)
+    images, tokens = co.synthetic_inputs(cfg, 2, seed=7)
+    model = rs.build_reference_clip(cfg, sd)
+    for sl in (-1, 0):
+        rts, ris = [], []
+        for b in range(2):
+            rt, ri = rs.reference_interpret(images[b:b + 1], tokens[b:b + 1], model, "cpu", sl, sl)
+            rts.append(rt.detach())
+            ris.append(ri.detach())
+        out[f"vit_b32.sl{sl}.R_text"], out[f"vit_b32.sl{sl}.R_image"] = torch.cat(rts).numpy(), torch.cat(ris).numpy()
+    del model, sd
+    cfg = co.SMALL
+    sd = co.init_state_dict(cfg, seed=4)
+    images, tokens = co.synthetic_inputs(cfg, 5, seed=9)
+    rt, ri = rs.reference_interpret(images[:1], tokens, rs.build_reference_clip(cfg, sd), "cpu", 0, 0)
+    out["repeat_small.R_text"], out["repeat_small.R_image"] = rt.detach().numpy(), ri.detach().numpy()
+    cfg = vo.VisualBertConfig(hidden=128, heads=8, intermediate=256, layers=4, vocab=80, max_pos=32, visual_dim=48, num_labels=31)
+    sd = vo.init_state_dict(cfg, 11)
+    inp = vo.synthetic_inputs(cfg, 2, 9, 12, seed=5)
+    for method in ("ours", "raw_attn", "rollout", "attn_gradcam"):
+        out["visualbert." + method] = ref_visualbert.generate(cfg, sd, inp, method).numpy()
+    cfg = do.DetrConfig(128, 4, 3, 3, 192, 9, 6)
+    sd = do.init_state_dict(cfg, 9)
+    src, pos, tq = do.synthetic_inputs(cfg, 2, 5, 6, seed=4)
+    out["detr_lrp"] = ref_detr.generate_ours(cfg, sd, src, pos, tq, use_lrp=True, normalize_self_attention=False).numpy()
+    cfg = lo.LxmertConfig(hidden=128, heads=4, intermediate=160, l_layers=3, x_layers=3, r_layers=2, vocab=70, max_pos=20,
+                          feat_dim=40, pos_dim=4, num_labels=17)
+    sd = lo.init_state_dict(cfg, 6)
+    ids, feats, boxes = lo.synthetic_inputs(cfg, 2, 9, 7, seed=3)
+    rtt, rti = ref_lxmert.generate_ours(cfg, sd, ids, feats, boxes, use_lrp=True)
+    out["lxmert_lrp.Rtt"], out["lxmert_lrp.Rti"] = rtt.numpy(), rti.numpy()
+    np.savez_compressed(os.path.join(OUT, "oracle_vs_reference.npz"), **out)
+    print("wrote oracle_vs_reference", {k: v.shape for k, v in out.items()})
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     argv = __import__("sys").argv
+    if "--vs-reference" in argv:
+        golden_vs_reference()
+        return
     if "--visualbert" in argv:
         golden_visualbert()
         return
@@ -279,6 +324,7 @@ def main():
     golden_lxmert_perturbation()
     golden_visualbert()
     golden_otsu()
+    golden_vs_reference()
 
 
 if __name__ == "__main__":

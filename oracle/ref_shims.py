@@ -1,8 +1,7 @@
 """Import shims that let the UNMODIFIED reference run on CPU in the build container.
 
-TEST INFRASTRUCTURE ONLY (see ``oracle/__init__.py``).  ``/root/reference`` exists only in the build container
-(never on the GPU box), so everything here is used by ``oracle/make_golden.py``,
-``tests/test_oracle_vs_reference.py`` (skipped when the tree is absent) and nothing else.
+TEST INFRASTRUCTURE ONLY (see ``oracle/__init__.py``).  The reference tree is needed only to regenerate the fixtures
+under ``tests/golden/``, so everything here is used by ``oracle/make_golden.py`` and nothing else.
 Shims (SURVEY.md §8c):
   * ``ftfy`` stub            - CLIP/clip/simple_tokenizer.py:6 imports it; the tokenizer is never called here.
   * ``Tensor.cuda`` identity - the reference hard-codes ``.cuda()`` (CLIP_explainability.ipynb:160,

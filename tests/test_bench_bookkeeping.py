@@ -34,6 +34,28 @@ def test_kernel_sources_hash_follows_code_not_comments():
     assert b.kernel_sources_hash("avg_heads", changed) == b.kernel_sources_hash("avg_heads")     # not one of its sources
 
 
+def test_dump_outputs_float32_and_seeded_sample_under_limit(tmp_path):
+    import numpy as np
+    import torch
+    b = _bench()
+    small = {"R_text": torch.randn(3, 4, 4, dtype=torch.float64), "R_image": np.arange(6).reshape(3, 2)}
+    b.dump_outputs(str(tmp_path / "small"), small)
+    for k, v in small.items():
+        got = np.load(tmp_path / "small" / f"{k}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, np.asarray(v, dtype=np.float32))
+    b.DUMP_LIMIT_BYTES = 100_000                          # this module instance only
+    n = 600
+    big = {"a": np.random.default_rng(1).random((n, 10, 10)), "b": np.arange(n, dtype=np.float32)[:, None]}
+    assert sum(v.size * 4 for v in big.values()) > b.DUMP_LIMIT_BYTES
+    for d in ("big1", "big2"):
+        b.dump_outputs(str(tmp_path / d), big)
+    a1, b1 = (np.load(tmp_path / "big1" / f"{k}.npy") for k in ("a", "b"))
+    assert a1.nbytes + b1.nbytes <= b.DUMP_LIMIT_BYTES and a1.shape[0] == b1.shape[0] > 0
+    keep = b1[:, 0].astype(int)                          # the same samples of every array, in order
+    assert np.all(np.diff(keep) > 0) and np.array_equal(a1, big["a"][keep].astype(np.float32))
+    assert np.array_equal(a1, np.load(tmp_path / "big2" / "a.npy"))
+
+
 def test_committed_traffic_capture_is_tied_to_kernel_sources():
     b = _bench()
     with open(os.path.join(ROOT, "profiles", "traffic_r2.json")) as f:

@@ -20,15 +20,20 @@ def _json_lines(out: str):
     return [json.loads(l) for l in out.splitlines() if l.startswith("{")]
 
 
-def test_reference_arm_single_process():
-    r = subprocess.run([sys.executable, "bench.py", "--impl", "reference", "--gpus", "1", "--steps", "1", "--warmup", "0"], cwd=ROOT,
-                       capture_output=True, text=True, timeout=540)
+def test_reference_arm_single_process(tmp_path):
+    r = subprocess.run([sys.executable, "bench.py", "--impl", "reference", "--gpus", "1", "--steps", "1", "--warmup", "0",
+                        "--dump-outputs", str(tmp_path)], cwd=ROOT, capture_output=True, text=True, timeout=540)
     assert r.returncode == 0, r.stderr[-2000:]
     (line,) = _json_lines(r.stdout)
     assert line["impl"] == "reference" and line["unit"] == "maps/s" and line["higher_is_better"] is True
     assert line["value"] > 0 and line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["value"] == line["value"] and line["e2e"]["h2d_bytes_per_step"] == 0
     assert line["config"]["workload"].startswith("clip_vit_b32")
+    import numpy as np
+    B, ctx = line["config"]["batch_per_gpu"], line["config"]["context"]
+    rt, ri = np.load(tmp_path / "R_text.npy"), np.load(tmp_path / "R_image.npy")
+    assert rt.shape == (B, ctx, ctx) and ri.shape == (B, 49) and rt.dtype == ri.dtype == np.float32
+    assert np.isfinite(rt).all() and np.isfinite(ri).all() and np.abs(ri).max() > 0
 
 
 def test_reference_arm_under_torchrun_prints_once():

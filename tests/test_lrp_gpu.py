@@ -196,11 +196,21 @@ def test_detr_r50_lrp_vs_oracle():
     sd = do.init_state_dict(cfg, seed=9)
     src, pos, tq = do.synthetic_inputs(cfg, 1, 6, 7, seed=4)
     r64 = do.generate_ours_lrp(sd, cfg, src, pos, tq, dtype=torch.float64)
-    ref_noise = rel_err(do.generate_ours_lrp(sd, cfg, src, pos, tq, dtype=torch.float32), r64)
+    # One fp32 evaluation is one draw of a heavy-tailed noise: its distance from fp64 ranges 0.013 .. 0.14 over CPU thread
+    # counts (summation orders) on one host.  The noise level is the median over four summation orders.
+    threads, draws = torch.get_num_threads(), []
+    try:
+        for n in (1, 2, 4, 8):
+            torch.set_num_threads(n)
+            draws.append(rel_err(do.generate_ours_lrp(sd, cfg, src, pos, tq, dtype=torch.float32), r64))
+    finally:
+        torch.set_num_threads(threads)
+    ref_noise = float(np.median(draws))
     eng = mmx_b200.DetrEngine(sd, nhead=cfg.nhead, device="cuda:0")
     out = mmx_b200.Generator(eng).generate_ours((src.cuda(), pos.cuda()), tq)
     e = rel_err(out.reshape(1, -1), r64)
-    print(f"DETR-R50 lrp vs fp64 oracle {e:.2e}; the reference algorithm in fp32 on this box vs fp64: {ref_noise:.2e}")
+    print(f"DETR-R50 lrp vs fp64 oracle {e:.2e}; the reference algorithm in fp32 vs fp64 at 1/2/4/8 threads: "
+          + " ".join(f"{x:.2e}" for x in draws))
     assert e < _bound(ref_noise)
     assert mmx_b200.lib().mmx_get_gemm_backend() != 0 or os.environ.get("MMX_GEMM_BACKEND") == "0"   # backend restored
 
